@@ -309,6 +309,16 @@ class Ranks:
             self.dist.destroy_process_group()
 
 
+def dump_outputs(dirpath, tensors):
+    """--dump-outputs: each tensor as DIR/<name>.npy, floats as float32, integers (indices) as float64, which holds
+    them exactly.  The largest dump, c5's [64, 131072] descriptors, is 34 MB."""
+    import numpy as np
+    os.makedirs(dirpath, exist_ok=True)
+    for name, t in tensors.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(dirpath, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 def collective_alone(R, shape, iters=10):
     """the step's all-gather timed on its own: -> (us per call, bus GB/s per rank = received bytes / time)"""
     torch, dist = R.torch, R.dist
@@ -401,9 +411,10 @@ def run_pipeline(args, wl):
 
     def loop(fn):
         def body(i):
-            fn(i)
+            out = fn(i)
             if i == loop.n - 1:
                 drain()                                             # every gather has landed inside the timed region
+                loop.last = out
         return body
 
     for i in range(args.warmup):
@@ -424,6 +435,8 @@ def run_pipeline(args, wl):
     ms_total = R.timed(loop(step_device), args.steps)               # un-instrumented: this is `value`
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"descriptors": loop.last})
 
     # end-to-end through the public API with host buffers (pinned), copies inside the timed region
     for i in range(max(1, args.warmup // 2)):
@@ -669,9 +682,15 @@ def run_retrieval(args, wl):
     if rank == 0:
         sampler.start()
     l0 = _lib.launch_count()
-    ms_total = R.timed(step, args.steps)
+    last = {}
+
+    def timed_step(i):
+        last["out"] = step(i)
+    ms_total = R.timed(timed_step, args.steps)
     launches = _lib.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:          # before any later call reuses the gather_db result buffers
+        dump_outputs(args.dump_outputs, {"distances": last["out"][0], "indices": last["out"][1]})
     for i in range(2):
         step_gather_queries(i)
         step_gather_db(i)
@@ -783,7 +802,12 @@ def main():
     ap.add_argument("--vocab", default="fit", choices=["fit", "random"])
     ap.add_argument("--precision", default="f16x3", choices=["f16x3", "tf32x3", "auto"],
                     help="operand pair format of the tensor-core GEMMs (both fp32-equivalent; see DESIGN.md)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned on rank 0 as DIR/<name>.npy (seeded inputs: two "
+                         "builds run with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference_arm(args, wl)

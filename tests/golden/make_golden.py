@@ -238,8 +238,77 @@ def make_build_vlads():
     print("build_vlads.npz")
 
 
+def make_reference_checks():
+    """The reference's VLAD.generate and get_top_k_recall, reduce_pca (both branches) and host helpers (to_pil_list,
+    pad_img, concat_desc_dists_clusters) on the seeded inputs of tests/util.py, which the tests regenerate."""
+    from tests import util as U
+    out = {}
+    vlads, db, qu, gt = U.vlad_topk_check_inputs()
+    for j, (x, c) in enumerate(vlads):
+        out[f"vlad{j}/out"] = ref_vlad(c.shape[0], c).generate(x).numpy()
+    d, i, r = ref.get_top_k_recall([1, 4], db, qu, gt)
+    out["topk/dist"], out["topk/idx"], out["topk/recalls"] = d.numpy(), i.numpy(), np.array([r[1], r[4]])
+    tr, te = U.pca_check_inputs()
+    for j, kw in enumerate(U.PCA_CHECK_KWARGS):
+        a = ref.reduce_pca(tr.copy(), te.copy(), 8, **kw)
+        out[f"pca{j}/train"], out[f"pca{j}/test"] = a[0], a[1]
+    c, x, img, batches = U.host_helper_inputs()
+    out["helpers/concat"] = ref.concat_desc_dists_clusters(c, x).numpy()
+    out["helpers/pad"] = ref.pad_img(img, 2, (255, 0, 3))
+    for b, batch in enumerate(batches):
+        for j, p in enumerate(ref.to_pil_list(batch)):
+            out[f"helpers/pil{b}_{j}"] = np.asarray(p)
+    np.savez_compressed(os.path.join(OUT, "reference_checks.npz"), **out)
+    print("reference_checks.npz")
+
+
+def make_dropin():
+    """What the reference's unmodified driver (`build_vlads`) leaves in its --cache-vlad-descs directory on the
+    synthetic dataset of tests/dropin_harness.py (hard and soft): the file list with each tensor's dtype and shape,
+    the vocabulary and assignments in full, the residual files as digests (tests/util.py).  Its descriptors equal
+    the uncached run's (build_vlads.npz).  Also the residual tensor of VLAD.generate_multi_res_vec, as a digest."""
+    import tempfile
+    from tests import dropin_harness as H
+    from tests import util as U
+    script = H.load_script(ref)
+    bv = U.load_cases("build_vlads.npz")
+    out = {}
+    for tag, soft in (("hard", False), ("soft", True)):
+        ds = H.SyntheticVprDataset()
+        with tempfile.TemporaryDirectory() as tmp, ri.hub_patched(H.hub_model):
+            np.random.seed(42)
+            largs = H.make_largs(script, tmp, H.MODEL, H.LAYER, "value", H.K, True, soft)
+            db, qu = script.build_vlads(largs, ds, verbose=False)
+            assert np.array_equal(db.numpy(), bv[tag]["db_vlads"]) and np.array_equal(qu.numpy(), bv[tag]["qu_vlads"])
+            cdir = H.cache_subdir(tmp)
+            meta = []
+            for dirpath, _, files in os.walk(cdir):
+                for f in files:
+                    rel = os.path.relpath(os.path.join(dirpath, f), cdir)
+                    t = torch.load(os.path.join(cdir, rel))
+                    meta.append(f"{rel}|{t.dtype}|{tuple(t.shape)}")
+                    if rel == "c_centers.pt":
+                        out[f"{tag}/c_centers"] = t.numpy()
+                    elif rel.endswith("_r.pt"):
+                        for k, v in U.digest(t.numpy()).items():
+                            out[f"{tag}/{rel[:-5]}_r_{k}"] = v
+                    else:
+                        out[f"{tag}/{rel[:-3]}"] = t.numpy()
+            out[f"{tag}/files"] = np.array(sorted(meta))
+    x, centers = H.residual_api_inputs()
+    with tempfile.TemporaryDirectory() as tmp:
+        torch.save(centers, os.path.join(tmp, "c_centers.pt"))
+        vr = ref.VLAD(5, cache_dir=tmp)
+        vr.fit(None)
+        for k, v in U.digest(vr.generate_multi_res_vec(x).numpy()).items():
+            out[f"residual_api/{k}"] = v
+    np.savez_compressed(os.path.join(OUT, "dropin.npz"), **out)
+    print("dropin.npz")
+
+
 if __name__ == "__main__":
     makers = {"vlad": make_vlad, "vlad_soft": make_vlad_soft, "fit": make_fit, "topk": make_topk,
-              "extract": make_extract, "preprocess": make_preprocess, "build_vlads": make_build_vlads}
+              "extract": make_extract, "preprocess": make_preprocess, "build_vlads": make_build_vlads,
+              "reference_checks": make_reference_checks, "dropin": make_dropin}
     for name in (sys.argv[1:] or list(makers)):      # `make_golden.py vlad_soft` regenerates one file
         makers[name]()

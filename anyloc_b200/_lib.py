@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libanyloc_b200.so")
 DIST = {"cosine": 0, "euclidean": 1}
 METRIC = {"cosine": 0, "l2": 1}
 FACET = {"query": 0, "key": 1, "value": 2, "token": 3}
+DESC = {"plain": 0, "l2": 1, "interleaved": 2}
 FFN = {"mlp": 0, "swiglufused": 1}
 EPI = {"bias": 0, "bias_split": 1, "gelu_split": 2, "swiglu_split": 3, "ls_resid": 4}
 ENGINE = {"auto": 0, "simt": 1, "tc3": 2}
@@ -27,7 +28,7 @@ class AnylocError(RuntimeError):
 
 class VitCfg(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("embed_dim", "depth", "num_heads", "ffn_kind", "ffn_hidden", "patch",
-                                       "pair_dtype")]
+                                       "pair_dtype", "stride")]
 
 
 _BLOCK_FIELDS = ["ln1_w", "ln1_b", "qkv_w_hi", "qkv_w_lo", "qkv_b", "proj_w_hi", "proj_w_lo", "proj_b",
@@ -92,6 +93,7 @@ _SIGS = {
     "anyloc_vit_extract": (C.c_int, [C.POINTER(VitCfg), C.POINTER(VitWeightsStruct), C.c_void_p,
                                      C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "anyloc_log_bin": (C.c_int, [C.c_void_p] + [C.c_int] * 5 + [C.c_void_p, C.c_void_p]),
     "anyloc_gemm_nt": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                  C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_void_p, C.c_void_p,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
@@ -178,7 +180,7 @@ class _WorkspacePool:
 
 workspaces = _WorkspacePool()
 
-PROF_CATEGORIES = ["gemm_tc", "gemm_simt", "attention", "layernorm", "vit_misc", "vlad", "topk"]
+PROF_CATEGORIES = ["gemm_tc", "gemm_simt", "attention", "layernorm", "vit_misc", "vlad", "topk", "log_bin"]
 
 
 def profile_enable(on=True):

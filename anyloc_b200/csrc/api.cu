@@ -1,6 +1,7 @@
 // C ABI of libanyloc_b200.so: error plumbing, building-block wrappers, GEMM engine dispatch and the
-// DINOv2 forward orchestration (early exit at the hooked module; reference
-// /root/reference/utilities.py:245-252,263-285 + upstream DinoVisionTransformer).
+// ViT forward orchestration (early exit at the hooked module; reference
+// /root/reference/utilities.py:245-252,263-285 + upstream DinoVisionTransformer for DINOv2, and
+// /root/reference/dino_extractor.py:190-332 + upstream DINO VisionTransformer for DINOv1).
 #include <stdarg.h>
 #include <string.h>
 #include <atomic>
@@ -58,10 +59,11 @@ bool gemm_tc_supported(const void* a_hi, const void* a_lo, int lda, const void* 
 // vit_ops.cu / attention.cu
 int launch_split(const float*, float*, float*, size_t, cudaStream_t);
 int launch_split_f16(const float*, void*, void*, size_t, float, cudaStream_t);
-int launch_im2col(const float*, int, int, int, int, int, void*, void*, bool, cudaStream_t);
+int launch_im2col(const float*, int, int, int, int, int, int, void*, void*, bool, cudaStream_t);
 int launch_assemble(const float*, const float*, const float*, int, int, int, float*, cudaStream_t);
 int launch_layernorm(const float*, const float*, const float*, int, int, float, void*, void*, bool, cudaStream_t);
 int launch_facet_out(const float*, int, int, int64_t, int, int, int, int, float*, cudaStream_t);
+int launch_facet_interleave(const float*, int, int, int64_t, int, int, int, float*, cudaStream_t);
 int launch_l2norm(const float*, int64_t, int, int64_t, float*, cudaStream_t);
 int attention_launch(const float*, const float*, int, int, int, int, void*, void*, bool, cudaStream_t);
 int attention_tc_launch(const float*, const float*, const float*, const float*, int, int, int, int, void*, void*, bool,
@@ -232,8 +234,14 @@ struct VitBuffers {
   float *pa_hi, *pa_lo, *ptmp, *x, *y_hi, *y_lo, *qkv, *qkv_lo, *vt_hi, *vt_lo, *h_hi, *h_lo;
   size_t vt_elems;
 };
+// patch grid of the (possibly overlapping) embedding conv: stride 0 means stride == patch
+int vit_stride(const AnylocVitCfg* c) { return c->stride ? c->stride : c->patch; }
+int vit_tokens(const AnylocVitCfg* c, int H, int W) {
+  const int S = vit_stride(c);
+  return (1 + (H - c->patch) / S) * (1 + (W - c->patch) / S);
+}
 size_t vit_carve(const AnylocVitCfg* c, int B, int H, int W, void* ws, size_t ws_bytes, VitBuffers* out) {
-  const int P = c->patch, N = (H / P) * (W / P), T = N + 1, D = c->embed_dim, Kp = anyloc_vit_patch_k(P);
+  const int P = c->patch, N = vit_tokens(c, H, W), T = N + 1, D = c->embed_dim, Kp = anyloc_vit_patch_k(P);
   const size_t M = (size_t)B * T;
   Workspace w(ws ? ws : (void*)256, ws ? ws_bytes : (size_t)-1 / 2);
   VitBuffers b;
@@ -252,7 +260,7 @@ size_t vit_carve(const AnylocVitCfg* c, int B, int H, int W, void* ws, size_t ws
 }  // namespace
 
 extern "C" size_t anyloc_vit_workspace_bytes(const AnylocVitCfg* cfg, int B, int H, int W) {
-  if (!cfg || B <= 0 || H < cfg->patch || W < cfg->patch) return 0;
+  if (!cfg || B <= 0 || cfg->patch <= 0 || cfg->stride < 0 || H < cfg->patch || W < cfg->patch) return 0;
   return vit_carve(cfg, B, H, W, nullptr, 0, nullptr) + 4096;
 }
 
@@ -296,17 +304,27 @@ static int vit_block(const AnylocVitCfg* c, const AnylocVitBlock& wb, const VitB
 
 extern "C" int anyloc_vit_extract(const AnylocVitCfg* cfg, const AnylocVitWeights* w, const float* img,
                                   int B, int H, int W, const float* pos_embed, int layer, int facet,
-                                  int use_cls, int norm_descs, float* out, void* ws, size_t ws_bytes,
+                                  int use_cls, int desc_mode, float* out, void* ws, size_t ws_bytes,
                                   int gemm_engine, void* stream) {
   ANYLOC_REQUIRE(cfg && w && img && pos_embed && out && ws, "vit_extract: null pointer");
-  ANYLOC_REQUIRE(cfg->patch > 0 && H % cfg->patch == 0 && W % cfg->patch == 0 && H > 0 && W > 0,
-                 "vit_extract: H=%d W=%d must be positive multiples of the patch size %d", H, W, cfg->patch);
+  if (cfg->stride == 0)
+    ANYLOC_REQUIRE(cfg->patch > 0 && H % cfg->patch == 0 && W % cfg->patch == 0 && H > 0 && W > 0,
+                   "vit_extract: H=%d W=%d must be positive multiples of the patch size %d", H, W, cfg->patch);
+  else
+    ANYLOC_REQUIRE(cfg->patch > 0 && cfg->stride > 0 && cfg->patch % cfg->stride == 0 && H >= cfg->patch &&
+                   W >= cfg->patch, "vit_extract: stride %d must divide the patch size %d and H=%d W=%d be >= it",
+                   cfg->stride, cfg->patch, H, W);
+  ANYLOC_REQUIRE(desc_mode >= ANYLOC_DESC_PLAIN && desc_mode <= ANYLOC_DESC_INTERLEAVED, "vit_extract: bad desc_mode %d",
+                 desc_mode);
+  if (desc_mode == ANYLOC_DESC_INTERLEAVED)
+    ANYLOC_REQUIRE(cfg->num_heads <= 16, "vit_extract: the interleaved layout supports at most 16 heads (got %d)",
+                   cfg->num_heads);
   ANYLOC_REQUIRE(layer >= 0 && layer < cfg->depth, "vit_extract: layer %d out of range [0,%d)", layer, cfg->depth);
   ANYLOC_REQUIRE(facet >= ANYLOC_FACET_QUERY && facet <= ANYLOC_FACET_TOKEN, "vit_extract: bad facet %d", facet);
   ANYLOC_REQUIRE(cfg->embed_dim == cfg->num_heads * 64, "vit_extract: head_dim must be 64");
   ANYLOC_REQUIRE(B > 0, "vit_extract: empty batch");
   cudaStream_t st = (cudaStream_t)stream;
-  const int P = cfg->patch, N = (H / P) * (W / P), T = N + 1, D = cfg->embed_dim, Kp = anyloc_vit_patch_k(P);
+  const int P = cfg->patch, N = vit_tokens(cfg, H, W), T = N + 1, D = cfg->embed_dim, Kp = anyloc_vit_patch_k(P);
   const int M = B * T;
   VitBuffers bf;
   if (!vit_carve(cfg, B, H, W, ws, ws_bytes, &bf)) {
@@ -322,7 +340,7 @@ extern "C" int anyloc_vit_extract(const AnylocVitCfg* cfg, const AnylocVitWeight
     ANYLOC_CHECK_CUDA(cudaMemsetAsync(bf.vt_lo, 0, bf.vt_elems * sizeof(float), st));
   }
   const bool f16 = cfg->pair_dtype == ANYLOC_PAIR_F16;
-  if ((rc = launch_im2col(img, B, H, W, P, Kp, bf.pa_hi, bf.pa_lo, f16, st))) return rc;
+  if ((rc = launch_im2col(img, B, H, W, P, vit_stride(cfg), Kp, bf.pa_hi, bf.pa_lo, f16, st))) return rc;
   EpiParams e_pe{ANYLOC_EPI_BIAS, w->patch_b, nullptr, nullptr, bf.ptmp, nullptr, D};
   e_pe.alpha = w->patch_alpha;
   if ((rc = gemm_dispatch(bf.pa_hi, bf.pa_lo, Kp, w->patch_w_hi, w->patch_w_lo, Kp, B * N, D, Kp, e_pe,
@@ -333,7 +351,7 @@ extern "C" int anyloc_vit_extract(const AnylocVitCfg* cfg, const AnylocVitWeight
   const AnylocVitBlock& wb = w->blocks[layer];
   if (facet == ANYLOC_FACET_TOKEN) {
     if ((rc = vit_block(cfg, wb, bf, B, T, gemm_engine, st))) return rc;
-    return launch_facet_out(bf.x, B, T, D, 0, D, use_cls, norm_descs, out, st);
+    return launch_facet_out(bf.x, B, T, D, 0, D, use_cls, desc_mode == ANYLOC_DESC_L2, out, st);
   }
   // q/k/v facet: only the requested third of the qkv projection of block `layer`
   if ((rc = launch_layernorm(bf.x, wb.ln1_w, wb.ln1_b, M, D, 1e-6f, bf.y_hi, bf.y_lo, f16, st))) return rc;
@@ -342,5 +360,6 @@ extern "C" int anyloc_vit_extract(const AnylocVitCfg* cfg, const AnylocVitWeight
   e_f.alpha = wb.qkv_alpha;
   if ((rc = gemm_dispatch(bf.y_hi, bf.y_lo, D, (const char*)wb.qkv_w_hi + woff,
                           (const char*)wb.qkv_w_lo + woff, D, M, D, D, e_f, gemm_engine, f16, st))) return rc;
-  return launch_facet_out(bf.qkv, B, T, D, 0, D, use_cls, norm_descs, out, st);
+  if (desc_mode == ANYLOC_DESC_INTERLEAVED) return launch_facet_interleave(bf.qkv, B, T, D, D, cfg->num_heads, use_cls, out, st);
+  return launch_facet_out(bf.qkv, B, T, D, 0, D, use_cls, desc_mode == ANYLOC_DESC_L2, out, st);
 }

@@ -110,7 +110,8 @@ static inline bool first_use_on_this_device(unsigned long long* seen) {
 void count_launch();
 
 // Optional per-category device timing (cudaEvents on the launching stream), see anyloc_profile_*.
-enum ProfCat { PC_GEMM_TC = 0, PC_GEMM_SIMT, PC_ATTENTION, PC_LAYERNORM, PC_VIT_MISC, PC_VLAD, PC_TOPK, PC_COUNT };
+enum ProfCat { PC_GEMM_TC = 0, PC_GEMM_SIMT, PC_ATTENTION, PC_LAYERNORM, PC_VIT_MISC, PC_VLAD, PC_TOPK, PC_LOG_BIN,
+               PC_COUNT };
 struct ProfScope {
   int slot; cudaStream_t st;
   ProfScope(int cat, cudaStream_t stream, double work);

@@ -1,8 +1,10 @@
 // Element-wise / row-wise pieces of the DINOv2 forward (upstream dinov2 DinoVisionTransformer,
-// reached from /root/reference/utilities.py:269): im2col for the 14x14/s14 patch embedding,
-// token assembly (+cls, +pos-embed), LayerNorm (eps 1e-6) fused with the tf32 (hi,lo) split
-// that feeds the tensor-core GEMMs, and the facet slice + F.normalize epilogue of
-// DinoV2ExtractFeatures.__call__ (utilities.py:270-283).
+// reached from /root/reference/utilities.py:269): im2col for the p x p / stride s patch embedding
+// (14/14 for DINOv2, 8 or 16 with stride p, p/2, p/4 for DINOv1's ViTExtractor), token assembly
+// (+cls, +pos-embed), LayerNorm (eps 1e-6) fused with the tf32 (hi,lo) split that feeds the
+// tensor-core GEMMs, the facet slice + F.normalize epilogue of DinoV2ExtractFeatures.__call__
+// (utilities.py:270-283) and the head-interleaved facet layout of ViTExtractor.extract_descriptors
+// (dino_extractor.py:329).
 #include "common.cuh"
 
 namespace anyloc {
@@ -32,11 +34,12 @@ template <> struct PairOut<true> {
   static __device__ __forceinline__ void put(__half* hi, __half* lo, size_t i, float v) { __half h, l; split_f16(v * kActScale, h, l); hi[i] = h; lo[i] = l; }
 };
 
-// img [B,3,H,W] -> patches (hi,lo) [B*gh*gw, Kp], column order (c, ky, kx) like conv weight.flatten(1)
+// img [B,3,H,W] -> patches (hi,lo) [B*gh*gw, Kp], column order (c, ky, kx) like conv weight.flatten(1).
+// Kernel P, stride S (S == P: the non-overlapping DINOv2 embedding), grid gh = 1 + (H-P)/S, gw = 1 + (W-P)/S.
 template <bool F16>
-__global__ void im2col_split_kernel(const float* __restrict__ img, int B, int H, int W, int P, int Kp,
+__global__ void im2col_split_kernel(const float* __restrict__ img, int B, int H, int W, int P, int S, int Kp,
                                     typename PairOut<F16>::T* __restrict__ hi, typename PairOut<F16>::T* __restrict__ lo) {
-  const int gh = H / P, gw = W / P;
+  const int gh = 1 + (H - P) / S, gw = 1 + (W - P) / S;
   const size_t row = blockIdx.x;               // patch index
   const int b = (int)(row / (gh * gw)), pi = (int)(row % (gh * gw));
   const int py = pi / gw, px = pi % gw;
@@ -45,7 +48,7 @@ __global__ void im2col_split_kernel(const float* __restrict__ img, int B, int H,
     float v = 0.f;
     if (c < Kreal) {
       int ch = c / (P * P), rem = c % (P * P), ky = rem / P, kx = rem % P;
-      v = __ldg(img + (((size_t)b * 3 + ch) * H + (py * P + ky)) * W + (px * P + kx));
+      v = __ldg(img + (((size_t)b * 3 + ch) * H + (py * S + ky)) * W + (px * S + kx));
     }
     PairOut<F16>::put(hi, lo, row * Kp + c, v);
   }
@@ -158,6 +161,41 @@ facet_out_kernel(const float* __restrict__ src, int B, int T, int64_t ld, int co
   }
 }
 
+// ViTExtractor's q/k/v layout: qkv[facet].permute(0,2,3,1).flatten(-2) of the [B,h,t,64] hook output puts channel
+// c = dd*heads + hd at projection column hd*64 + dd.  One warp per token row: the row is read coalesced (float4) into
+// shared memory as [heads][65] (the pad keeps the column gather below conflict-free), then written coalesced (float4)
+// in the interleaved order.  No normalisation (extract_descriptors returns raw facets).
+__global__ void __launch_bounds__(256)
+facet_interleave_kernel(const float* __restrict__ src, int B, int T, int64_t ld, int D, int heads, int use_cls,
+                        float* __restrict__ out) {
+  extern __shared__ float sm_rows[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int Tout = use_cls ? T : T - 1;
+  const int64_t row = (int64_t)blockIdx.x * 8 + warp;
+  if (row >= (int64_t)B * Tout) return;
+  float* s = sm_rows + warp * heads * 65;
+  const int b = (int)(row / Tout), t = (int)(row % Tout) + (use_cls ? 0 : 1);
+  const float4* xr = reinterpret_cast<const float4*>(src + ((int64_t)b * T + t) * ld);
+  const int D4 = D >> 2;
+  for (int d4 = lane; d4 < D4; d4 += 32) {
+    const float4 v = xr[d4];
+    const int d = d4 << 2;
+    float* p = s + (d >> 6) * 65 + (d & 63);      // four columns of one head (64 % 4 == 0)
+    p[0] = v.x; p[1] = v.y; p[2] = v.z; p[3] = v.w;
+  }
+  __syncwarp();
+  float4* yr = reinterpret_cast<float4*>(out + row * D);
+  for (int c4 = lane; c4 < D4; c4 += 32) {
+    float r[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int c = (c4 << 2) + j, dd = c / heads, hd = c - dd * heads;
+      r[j] = s[hd * 65 + dd];
+    }
+    yr[c4] = make_float4(r[0], r[1], r[2], r[3]);
+  }
+}
+
 int launch_split(const float* x, float* hi, float* lo, size_t n, cudaStream_t st) {
   int blocks = (int)std::min<size_t>((n + 255) / 256, (size_t)device_sm_count() * 16);
   if (blocks < 1) blocks = 1;
@@ -172,9 +210,11 @@ int launch_split_f16(const float* x, void* hi, void* lo, size_t n, float scale, 
   ANYLOC_CHECK_LAUNCH();
   return ANYLOC_OK;
 }
-int launch_im2col(const float* img, int B, int H, int W, int P, int Kp, void* hi, void* lo, bool f16, cudaStream_t st) {
-  if (f16) im2col_split_kernel<true><<<B * (H / P) * (W / P), 128, 0, st>>>(img, B, H, W, P, Kp, (__half*)hi, (__half*)lo);
-  else im2col_split_kernel<false><<<B * (H / P) * (W / P), 128, 0, st>>>(img, B, H, W, P, Kp, (float*)hi, (float*)lo);
+int launch_im2col(const float* img, int B, int H, int W, int P, int S, int Kp, void* hi, void* lo, bool f16,
+                  cudaStream_t st) {
+  const int rows = B * (1 + (H - P) / S) * (1 + (W - P) / S);
+  if (f16) im2col_split_kernel<true><<<rows, 128, 0, st>>>(img, B, H, W, P, S, Kp, (__half*)hi, (__half*)lo);
+  else im2col_split_kernel<false><<<rows, 128, 0, st>>>(img, B, H, W, P, S, Kp, (float*)hi, (float*)lo);
   ANYLOC_CHECK_LAUNCH();
   return ANYLOC_OK;
 }
@@ -205,6 +245,14 @@ int launch_facet_out(const float* src, int B, int T, int64_t ld, int col0, int D
                      float* out, cudaStream_t st) {
   int64_t rows = (int64_t)B * (use_cls ? T : T - 1);
   facet_out_kernel<<<(int)((rows + 7) / 8), 256, 0, st>>>(src, B, T, ld, col0, D, use_cls, do_norm, out);
+  ANYLOC_CHECK_LAUNCH();
+  return ANYLOC_OK;
+}
+int launch_facet_interleave(const float* src, int B, int T, int64_t ld, int D, int heads, int use_cls, float* out,
+                            cudaStream_t st) {
+  int64_t rows = (int64_t)B * (use_cls ? T : T - 1);
+  facet_interleave_kernel<<<(int)((rows + 7) / 8), 256, 8 * heads * 65 * sizeof(float), st>>>(src, B, T, ld, D, heads,
+                                                                                              use_cls, out);
   ANYLOC_CHECK_LAUNCH();
   return ANYLOC_OK;
 }

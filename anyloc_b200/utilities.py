@@ -276,7 +276,64 @@ class _HookHandle:
         pass
 
 
-class DinoV2ExtractFeatures:
+class _PrecisionPolicy:
+    """How an extractor feeds fp32 operands to the tensor cores, shared by DinoV2ExtractFeatures and the DINOv1
+    ViTExtractor (anyloc_b200/dino_v1.py): "tf32x3", "f16x3" or "auto" (see DinoV2ExtractFeatures).  Subclasses
+    provide `_make_weights(state_dict, pair)` -> vit.VitWeights and run every forward through `_run_guarded`."""
+
+    _OVERFLOW_MSG = ("f16x3 precision overflowed the fp16 operand range (|8*x| > 65504 somewhere in the network); "
+                     "construct the extractor with precision='tf32x3' (or 'auto')")
+
+    def _init_precision(self, precision, state_dict):
+        precision = precision or os.environ.get("ANYLOC_B200_PRECISION", "auto")
+        if precision not in ("tf32x3", "f16x3", "auto"):
+            raise ValueError(f"precision must be 'auto', 'tf32x3' or 'f16x3', got {precision!r}")
+        self._auto = precision == "auto"
+        self._state_dict = state_dict if self._auto else None     # kept for the tf32x3 re-upload on an overflow
+        self.precision = "f16x3" if self._auto else precision
+        self._vit = self._make_weights(state_dict, "f16" if self.precision == "f16x3" else "tf32")
+        # fp16-range guard of the f16x3 format: "sync" = checked before a call returns (one host sync per call),
+        # "deferred" = the flag of call i is read at call i+1 / raise_if_overflowed() (no sync on the hot loop),
+        # "off".  precision="auto" always checks synchronously (it has to decide before returning).
+        self.check_finite = os.environ.get("ANYLOC_B200_CHECK_FINITE", "sync")
+        if self.check_finite in ("1", "0"):
+            self.check_finite = "sync" if self.check_finite == "1" else "off"
+        self._pending_flag = None
+
+    def raise_if_overflowed(self):
+        """Deferred mode: reads the finite-flag of the last call (one host sync)."""
+        flag, self._pending_flag = self._pending_flag, None
+        if flag is not None and not bool(flag):
+            raise _lib.AnylocError(self._OVERFLOW_MSG)
+
+    def _switch_to_tf32(self):
+        print("anyloc_b200: f16x3 operands overflowed the fp16 range -- switching this extractor to tf32x3 "
+              "(full fp32 exponent range, ~2x slower)")
+        self._vit = None
+        torch.cuda.empty_cache()
+        self._vit = self._make_weights(self._state_dict, "tf32")
+        self.precision, self._auto, self._state_dict = "tf32x3", False, None
+
+    def _run_guarded(self, run):
+        """run(VitWeights) -> device tensor, checked against the fp16 range as configured"""
+        if self.check_finite == "deferred" and not self._auto:
+            self.raise_if_overflowed()
+        out = run(self._vit)
+        if self.precision != "f16x3" or (self.check_finite == "off" and not self._auto):
+            return out
+        flag = torch.isfinite(out).all()
+        if self.check_finite == "deferred" and not self._auto:
+            self._pending_flag = flag
+            return out
+        if bool(flag):
+            return out
+        if not self._auto:
+            raise _lib.AnylocError(self._OVERFLOW_MSG)
+        self._switch_to_tf32()
+        return run(self._vit)
+
+
+class DinoV2ExtractFeatures(_PrecisionPolicy):
     """Extract features from an intermediate layer of DINOv2 (utilities.py:219-288).
 
     Same constructor and call signature.  The forward stops at the hooked module (blocks
@@ -297,71 +354,32 @@ class DinoV2ExtractFeatures:
                  gemm_engine: str = "auto", precision: str = None) -> None:
         self.vit_type: str = dino_model
         self.device = torch.device(device)
-        dev = _lib.require_cuda(self.device)
+        self._dev = _lib.require_cuda(self.device)
         if facet not in _lib.FACET:
             raise ValueError(f"facet must be one of {sorted(_lib.FACET)}, got {facet!r}")
-        sd = weights if weights is not None else _vit.resolve_state_dict(dino_model, dev)
-        # only blocks 0..layer are ever executed (early exit), so only those are uploaded
-        precision = precision or os.environ.get("ANYLOC_B200_PRECISION", "auto")
-        if precision not in ("tf32x3", "f16x3", "auto"):
-            raise ValueError(f"precision must be 'auto', 'tf32x3' or 'f16x3', got {precision!r}")
-        self._auto = precision == "auto"
-        self._state_dict = sd if self._auto else None     # kept for the tf32x3 re-upload on an fp16-range overflow
-        self.precision = "f16x3" if self._auto else precision
-        self.dino_model = _vit.VitWeights(dino_model, sd, dev, depth=layer + 1,
-                                          pair="f16" if self.precision == "f16x3" else "tf32")
+        sd = weights if weights is not None else _vit.resolve_state_dict(dino_model, self._dev)
         self.layer: int = layer
+        self._init_precision(precision, sd)
         self.facet = facet
         self.use_cls = use_cls
         self.norm_descs = norm_descs
         self.gemm_engine = gemm_engine
         self.fh_handle = _HookHandle()
         self._hook_out = None
-        # fp16-range guard of the f16x3 format: "sync" = checked before __call__ returns (one host sync per call),
-        # "deferred" = the flag of call i is read at call i+1 / raise_if_overflowed() (no sync on the hot loop),
-        # "off".  precision="auto" always checks synchronously (it has to decide before returning).
-        self.check_finite = os.environ.get("ANYLOC_B200_CHECK_FINITE", "sync")
-        if self.check_finite in ("1", "0"):
-            self.check_finite = "sync" if self.check_finite == "1" else "off"
-        self._pending_flag = None
 
-    _OVERFLOW_MSG = ("f16x3 precision overflowed the fp16 operand range (|8*x| > 65504 somewhere in the network); "
-                     "construct the extractor with precision='tf32x3' (or 'auto')")
+    @property
+    def dino_model(self):
+        """the device-resident backbone (vit.VitWeights)"""
+        return self._vit
 
-    def raise_if_overflowed(self):
-        """Deferred mode: reads the finite-flag of the last call (one host sync)."""
-        flag, self._pending_flag = self._pending_flag, None
-        if flag is not None and not bool(flag):
-            raise _lib.AnylocError(self._OVERFLOW_MSG)
-
-    def _switch_to_tf32(self):
-        print("anyloc_b200: f16x3 operands overflowed the fp16 range -- switching this extractor to tf32x3 "
-              "(full fp32 exponent range, ~2x slower)")
-        dev, name = self.dino_model.device, self.dino_model.name
-        self.dino_model = None
-        torch.cuda.empty_cache()
-        self.dino_model = _vit.VitWeights(name, self._state_dict, dev, depth=self.layer + 1, pair="tf32")
-        self.precision, self._auto, self._state_dict = "tf32x3", False, None
+    def _make_weights(self, state_dict, pair):
+        # only blocks 0..layer are ever executed (early exit), so only those are uploaded
+        return _vit.VitWeights(self.vit_type, state_dict, self._dev, depth=self.layer + 1, pair=pair)
 
     def __call__(self, img: torch.Tensor) -> torch.Tensor:
         with torch.no_grad():
-            if self.check_finite == "deferred" and not self._auto:
-                self.raise_if_overflowed()
-            out = self.dino_model.extract(img, self.layer, self.facet, self.use_cls, self.norm_descs,
-                                          self.gemm_engine)
-            if self.precision != "f16x3" or (self.check_finite == "off" and not self._auto):
-                return out
-            flag = torch.isfinite(out).all()
-            if self.check_finite == "deferred" and not self._auto:
-                self._pending_flag = flag
-                return out
-            if bool(flag):
-                return out
-            if not self._auto:
-                raise _lib.AnylocError(self._OVERFLOW_MSG)
-            self._switch_to_tf32()
-            return self.dino_model.extract(img, self.layer, self.facet, self.use_cls, self.norm_descs,
-                                           self.gemm_engine)
+            return self._run_guarded(lambda m: m.extract(img, self.layer, self.facet, self.use_cls, self.norm_descs,
+                                                         self.gemm_engine))
 
     def __del__(self):
         pass

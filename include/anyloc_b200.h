@@ -41,7 +41,12 @@ extern "C" {
 #define ANYLOC_FACET_KEY 1
 #define ANYLOC_FACET_VALUE 2
 #define ANYLOC_FACET_TOKEN 3
-/* ffn kinds of the DINOv2 family (upstream dinov2/hub/backbones.py) */
+/* desc_mode of anyloc_vit_extract: how the selected facet rows are written */
+#define ANYLOC_DESC_PLAIN 0        /* rows as computed (DinoV2ExtractFeatures norm_descs=False)                */
+#define ANYLOC_DESC_L2 1           /* rows / max(|row|,1e-12)  (norm_descs=True)                              */
+#define ANYLOC_DESC_INTERLEAVED 2 /* ViTExtractor layout (dino_extractor.py:329): q/k/v channel c = dd*heads + h
+                                      reads projection column h*64 + dd; token rows plain; no normalisation     */
+/* ffn kinds of the DINOv2 family (upstream dinov2/hub/backbones.py); DINOv1 uses ANYLOC_FFN_MLP */
 #define ANYLOC_FFN_MLP 0
 #define ANYLOC_FFN_SWIGLU 1
 
@@ -71,10 +76,10 @@ int anyloc_device_info(int* sm_count, size_t* smem_optin_bytes);
  * anyloc_launch_count: kernels launched by this library since load (all threads).
  * Profiling (off by default; not thread-safe): when enabled every launch group records a cudaEvent
  * pair on its stream; anyloc_profile_read synchronises them and returns, per category
- * (0 gemm_tc, 1 gemm_simt, 2 attention, 3 layernorm, 4 vit_misc, 5 vlad, 6 topk), the summed
+ * (0 gemm_tc, 1 gemm_simt, 2 attention, 3 layernorm, 4 vit_misc, 5 vlad, 6 topk, 7 log_bin), the summed
  * device milliseconds, the number of launch groups and the summed algorithmic work
  * (FLOPs for 0-2, bytes otherwise), then clears the records. */
-#define ANYLOC_PROF_CATEGORIES 7
+#define ANYLOC_PROF_CATEGORIES 8
 long long anyloc_launch_count(void);
 int anyloc_profile_enable(int on);
 int anyloc_profile_read(double* ms, long long* groups, double* work);
@@ -181,6 +186,9 @@ int anyloc_allgather_desc(void* nccl_comm, const float* local, float* all, size_
  * Replaces DinoV2ExtractFeatures.__call__ (utilities.py:263-285) and the hub model's forward
  * it triggers (facebookresearch/dinov2 DinoVisionTransformer, see SURVEY.md App. A), with the
  * early exit at the hooked module (blocks 0..layer-1, then norm1+qkv-third or the whole block).
+ * The same forward serves DINOv1 (dino_extractor.py:ViTExtractor, facebookresearch/dino): its
+ * blocks are the DINOv2 MLP blocks without LayerScale (pass ones for ls1/ls2), and its patch
+ * embedding may be overlapping (stride < patch).
  */
 typedef struct {
   int embed_dim;   /* 384 / 768 / 1024 / 1536 */
@@ -188,8 +196,11 @@ typedef struct {
   int num_heads;   /* head_dim must be 64 */
   int ffn_kind;    /* ANYLOC_FFN_* */
   int ffn_hidden;  /* 4*D (mlp) or 4096-style fused hidden (swiglu) */
-  int patch;       /* 14 */
+  int patch;       /* 14 (DINOv2), 8 or 16 (DINOv1) */
   int pair_dtype;  /* ANYLOC_PAIR_*: format of the weight pairs and of all GEMM-input activations */
+  int stride;      /* patch-embedding conv stride: 0 = patch with H, W multiples of the patch; otherwise a divisor
+                      of the patch, grid gh = 1 + (H-patch)/stride, gw = 1 + (W-patch)/stride (trailing pixels
+                      dropped, like the strided Conv2d of dino_extractor.py:141-160) */
 } AnylocVitCfg;
 
 /* Per-block device pointers.  Matrices are [out,in] row-major like nn.Linear.weight, supplied as
@@ -216,15 +227,24 @@ typedef struct {
   float patch_alpha;
 } AnylocVitWeights;
 
-/* padded patch-embed reduction length (3*14*14=588 -> multiple of 32) */
+/* padded patch-embed reduction length (3*14*14=588 -> multiple of 32; 192 / 768 for patch 8 / 16) */
 int anyloc_vit_patch_k(int patch);
 size_t anyloc_vit_workspace_bytes(const AnylocVitCfg* cfg, int B, int H, int W);
-/* img [B,3,H,W] fp32 (H,W multiples of 14); pos_embed [1+g_h*g_w, D] already interpolated for this
- * grid (upstream interpolate_pos_encoding); out [B, N(+1 if use_cls), D]. */
+/* img [B,3,H,W] fp32 (see AnylocVitCfg.stride for the admissible H, W); pos_embed [1+g_h*g_w, D] already
+ * interpolated for this grid (upstream interpolate_pos_encoding); out [B, N(+1 if use_cls), D].
+ * desc_mode: ANYLOC_DESC_* (0/1 are DinoV2ExtractFeatures' norm_descs). */
 int anyloc_vit_extract(const AnylocVitCfg* cfg, const AnylocVitWeights* w_host, const float* img,
                        int B, int H, int W, const float* pos_embed, int layer, int facet,
-                       int use_cls, int norm_descs, float* out, void* ws, size_t ws_bytes,
+                       int use_cls, int desc_mode, float* out, void* ws, size_t ws_bytes,
                        int gemm_engine, void* stream);
+
+/* Log-binned descriptor of ViTExtractor._log_bin (dino_extractor.py:260-306), hierarchy 2 (the only one any
+ * caller uses; others return ANYLOC_ERR_UNSUPPORTED).  x [B, gh*gw, C] fp32 (row-major grid, C % 4 == 0) ->
+ * out [B, gh*gw, 17*C], bin-major (bin*C + c):
+ *   bins 0-8   x  at (clamp(y+dy), clamp(x+dx)),     dy,dx in {-1,0,1} row-major
+ *   bins 9-16  A1 at (clamp(y+3dy), clamp(x+3dx)),   centre skipped
+ * A1 = 3x3 average, stride 1, padding 1, count_include_pad=False (AvgPool2d). */
+int anyloc_log_bin(const float* x, int B, int gh, int gw, int C, int hierarchy, float* out, void* stream);
 
 /* ------------------------------------------- building blocks (exported for parity tests)
  * C[M,N] = (A_hi+A_lo)[M,K] . (B_hi+B_lo)[N,K]^T with epilogue; *_lo nullable (treated as 0).
